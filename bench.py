@@ -2,6 +2,7 @@
 """Benchmark of the cross-attention heat-map hot path (BASELINE.json metric: heat-map px/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload sd21|sd21_768|sdxl|sdxl70|sd15] [--prompts P]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): random-init SD-2.1-base UNet shapes, 64x64 latent, 77 tokens, bf16, the 15 traced
 cross-attention layers of one denoising step. A bench "step" is one pass of the hot path over one step's Q/K:
@@ -215,12 +216,12 @@ def build_sets(layers, n_prompts, dtype, n_sets, seed):
 
 
 def leg_value(args, layers, dtype, D: Dist, windows):
-    """K steps (one persistent launch per traced-layer pack each) between CUDA events, repeated over R blocks.
+    """K steps (one persistent launch per traced-layer pack each) between CUDA events: barrier + synchronize, K timed
+    steps, synchronize + barrier; the time is the max over ranks. The launches are queued behind a short spin kernel so
+    that the device executes them back to back: the figure is device throughput, not host launch pacing (8 Python
+    processes share one host at N=8).
 
-    Every block is what the contract describes -- barrier + synchronize, K timed steps, synchronize + barrier -- and the
-    reported time is the median block (max over ranks per block). The launches of a block are queued behind a short
-    spin kernel so that the device executes them back to back: the figure is device throughput, not host launch pacing
-    (8 Python processes share one host at N=8)."""
+    Also returns the accumulators of the prompt set the last timed step added into: what the caller of the path gets."""
     from daam_b200 import _native, ops
     n_sets, _ = value_sets(layers, args.prompts)               # working set >= 320 MB > 126 MB L2
     sets = build_sets(layers, args.prompts, dtype, n_sets, 1234 + D.rank)
@@ -229,51 +230,41 @@ def leg_value(args, layers, dtype, D: Dist, windows):
     for i in range(args.warmup):
         ops.accumulate(sets[i % n_sets][0], 'cuda', stream, flags)
     torch.cuda.synchronize()
-    blocks = max(10, -(-200 // args.steps))
     gate_cycles = int(max(2.0, args.steps * 0.04) * 1.9e6)     # ~max(2 ms, 40 us per launch) at 1.9 GHz
     launches0 = _native.launch_count()
-    block_ms, step = [], args.warmup
-    for _ in range(blocks):
-        D.barrier()
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        t0 = time.time()
-        torch.cuda._sleep(gate_cycles)
-        e0.record(stream)
-        for _k in range(args.steps):
-            ops.accumulate(sets[step % n_sets][0], 'cuda', stream, flags)
-            step += 1
-        e1.record(stream)
-        torch.cuda.synchronize()
-        D.barrier()
-        torch.cuda.synchronize()
-        block_ms.append(e0.elapsed_time(e1))
-        if len(block_ms) == 1:
-            t_first = t0
-    windows.append((t_first, time.time()))
-    launches = (_native.launch_count() - launches0) // blocks          # per K-step block
-    mine = torch.tensor(block_ms, dtype=torch.float64, device='cuda')
+    step = args.warmup
+    D.barrier()
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    t0 = time.time()
+    torch.cuda._sleep(gate_cycles)
+    e0.record(stream)
+    for _k in range(args.steps):
+        ops.accumulate(sets[step % n_sets][0], 'cuda', stream, flags)
+        step += 1
+    e1.record(stream)
+    torch.cuda.synchronize()
+    D.barrier()
+    torch.cuda.synchronize()
+    windows.append((t0, time.time()))
+    launches = _native.launch_count() - launches0
+    mine = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device='cuda')
     if D.world > 1:
-        allr = torch.empty(D.world, blocks, dtype=torch.float64, device='cuda')
-        D.dist.all_gather_into_tensor(allr, mine.unsqueeze(0))
+        allr = torch.empty(D.world, dtype=torch.float64, device='cuda')
+        D.dist.all_gather_into_tensor(allr, mine)
     else:
-        allr = mine.unsqueeze(0)
-    per_block_max = allr.max(dim=0).values                              # max over ranks, block by block
-    ms = float(per_block_max.median())
-    us = allr / args.steps * 1e3                                        # per-launch-step, per rank and block
-    stats = {'blocks': blocks, 'steps_per_block': args.steps,
-             'us_per_step_median_block_max_over_ranks': round(ms / args.steps * 1e3, 3),
-             'us_per_step_best_block_max_over_ranks': round(float(per_block_max.min()) / args.steps * 1e3, 3),
-             'us_per_step_worst_block_max_over_ranks': round(float(per_block_max.max()) / args.steps * 1e3, 3),
-             'per_rank_us_per_step': [{'rank': r, 'min': round(float(us[r].min()), 3),
-                                       'median': round(float(us[r].median()), 3), 'max': round(float(us[r].max()), 3)}
+        allr = mine
+    ms = float(allr.max())
+    stats = {'steps': args.steps, 'us_per_step_max_over_ranks': round(ms / args.steps * 1e3, 3),
+             'per_rank_us_per_step': [{'rank': r, 'us': round(float(allr[r]) / args.steps * 1e3, 3)}
                                       for r in range(D.world)]}
     # sanity: the timed work really accumulated (softmax rows sum to 1 -> each head gained hw per visit)
     q, k, acc = sets[0][1][0]
     visits = len(range(0, step, n_sets))
     got = float(acc[0, 0].double().sum())
     assert abs(got - visits * acc.shape[-1]) < 1e-3 * got, (got, visits)
-    return ms, launches, n_sets, stats
+    last = [acc for _, _, acc in sets[(step - 1) % n_sets][1]]
+    return ms, launches, n_sets, stats, last
 
 
 def leg_e2e(args, spec, dtype, D: Dist, windows, cuda_graph=True):
@@ -336,7 +327,7 @@ def leg_e2e(args, spec, dtype, D: Dist, windows, cuda_graph=True):
             order = {'ok': False, 'error': repr(e)}
         if not order['ok']:
             log(f'[bench] WARNING: gather order check failed: {order}')
-    return ms, h2d, d2h, order
+    return ms, h2d, d2h, order, out_h
 
 
 def leg_hook_overhead(args, spec, dtype, windows):
@@ -547,6 +538,26 @@ def run_reference(args):
     emit(line)
 
 
+DUMP_BYTES = 63_000_000   # data of all dumped arrays together, .npy headers aside: under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of ``arrays`` (name -> tensor) as ``<out_dir>/<name>.npy`` in float32. When they exceed
+    DUMP_BYTES together, each is replaced by the same share of its elements at positions drawn from a fixed seed (the
+    same positions on every run), flattened."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() for t in arrays.values()) * 4
+    share = min(1.0, DUMP_BYTES / total)
+    for i, (name, t) in enumerate(arrays.items()):
+        t = t.detach().float()
+        if share < 1.0:
+            idx = torch.randint(t.numel(), (int(t.numel() * share),), generator=torch.Generator().manual_seed(i))
+            t = t.flatten()[idx.sort().values.to(t.device)]
+        np.save(os.path.join(out_dir, f'{name}.npy'), t.cpu().numpy())
+    log(f'[bench] wrote {len(arrays)} arrays to {out_dir}' + (f' ({share:.3f} of each, seeded sample)' if share < 1 else ''))
+
+
 def workload_spec(workload):
     from daam_b200.testing.synthetic import SD15_SPEC, SD21_768_SPEC, SD21_SPEC, SDXL_SPEC
     return {'sd21': SD21_SPEC, 'sd21_768': SD21_768_SPEC, 'sdxl': SDXL_SPEC, 'sdxl70': SDXL_SPEC, 'sd15': SD15_SPEC}[workload]
@@ -571,7 +582,6 @@ def value_sets(layers, prompts):
 def shared_config(args, layers, world):
     """The `config` object: identical for both arms of a run (the reference arm runs `on your arm's config`)."""
     n_sets, set_bytes = value_sets(layers, args.prompts)
-    blocks = max(10, -(-200 // args.steps))
     return {
         'workload': workload_name(args), 'px_per_step': px_per_step(layers, args.prompts),
         'px_definition': 'sum over traced layers of heads*77*h*w',
@@ -579,8 +589,8 @@ def shared_config(args, layers, world):
         'l2': f'inputs larger than L2: steps rotate over {n_sets} resident prompt sets '
               f'({n_sets * set_bytes / 1e6:.0f} MB of accumulators+Q/K vs 126 MB L2), no flush',
         'launch': 'one persistent kernel per step per pack of <= 32 traced layers',
-        'timing': f'value: median of {blocks} blocks of K={args.steps} steps (each block between barrier+synchronize, '
-                  f'CUDA events, max over ranks; launches queued behind a spin kernel so host pacing is not timed)',
+        'timing': f'value: K={args.steps} steps between barrier+synchronize, CUDA events, max over ranks; launches '
+                  f'queued behind a spin kernel so host pacing is not timed',
         'parallelism': f'prompts sharded, dp{world}',
     }
 
@@ -601,7 +611,14 @@ def main():
     ap.add_argument('--skip-cpu', action='store_true')
     ap.add_argument('--skip-eager', action='store_true', help='skip the eager (no CUDA graph) e2e leg')
     ap.add_argument('--skip-e2e', action='store_true', help='kernel legs only (profiling runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what they computed as DIR/<name>.npy (float32, <= 64 MB): the '
+                         'accumulators of the last timed step\'s prompt set and the e2e leg\'s heat maps (rank 0)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'daam_b200':
+        ap.error('--dump-outputs writes the outputs of --impl daam_b200')
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.dtype is None:   # sd15: the reference's default load
         args.dtype = {'sd21': 'bf16', 'sd21_768': 'bf16', 'sdxl': 'fp16', 'sdxl70': 'fp16', 'sd15': 'fp32'}[args.workload]
     args.warmup = max(3, args.warmup)
@@ -621,14 +638,18 @@ def main():
     windows = []
 
     with torch.no_grad():
-        ms, launches, n_sets, value_stats = leg_value(args, layers, dtype, D, windows)
+        ms, launches, n_sets, value_stats, last_accs = leg_value(args, layers, dtype, D, windows)
+        outputs = {f'accumulator_layer{i:02d}': acc for i, acc in enumerate(last_accs)}
         e2e_ms = eager_ms = float('nan')
         h2d = d2h = 0
         order = None
         if not args.skip_e2e:
-            e2e_ms, h2d, d2h, order = leg_e2e(args, spec, dtype, D, windows, cuda_graph=True)
+            e2e_ms, h2d, d2h, order, outputs['e2e_heat_maps'] = leg_e2e(args, spec, dtype, D, windows, cuda_graph=True)
             if not args.skip_eager:
                 eager_ms = leg_e2e(args, spec, dtype, D, windows, cuda_graph=False)[0]
+        if args.dump_outputs and D.rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
+        del outputs, last_accs
         overhead = None
         if not args.skip_overhead:       # every rank measures its own GPU (all ranks share the host's cores)
             try:

@@ -5,10 +5,10 @@ Nothing in the product (``daam_b200/``) imports this file. Only ``tests/``, ``__
 baseline -- never as the thing shipped.
 
 Parity status: the reference holds no tests, golden vectors or fixtures for this path (SURVEY.md section 4 / section 8c), so
-the oracle is pinned the other way the task allows: against outputs of the reference itself. ``tests/
-test_oracle_vs_reference.py`` runs the *verbatim* reference (imported from ``/root/reference`` behind the stubs in
-``oracle/ref_loader.py``) and this restatement on identical seeded inputs and requires bit-equality on CPU fp32;
-``oracle/make_golden.py`` stores reference outputs as fixtures under ``tests/golden/`` that travel to the GPU box.
+the oracle is pinned the other way the task allows: against outputs of the reference itself. ``oracle/make_golden.py``
+runs the *verbatim* reference (imported behind the stubs in ``oracle/ref_loader.py``) on seeded inputs and stores what it
+computed as fixtures under ``tests/golden/``; ``tests/test_oracle_vs_reference.py`` runs this restatement on the same
+inputs and requires bit-equality on CPU fp32.
 
 Two layers live here:
 

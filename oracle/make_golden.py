@@ -18,6 +18,13 @@ Fixtures
                      (96, 96) global maps from keys at 96^2 / 48^2 / 24^2.
   perkey.npz         the reference's --all-heads sweep (daam/run/generate.py:239-255) over finalize.npz's keys:
                      ``compute_global_heat_map(layer_idx=l, head_idx=h)`` for every key, plain and normalised.
+  reference_trace.npz what tests/test_oracle_vs_reference.py compares the oracle with: the reference's per-key
+                     accumulators, heat maps, saved heads and error messages of its scenarios, as exact bit fingerprints
+                     (tests/util.py ``fingerprint``), single-threaded. The same generation's global maps are in
+                     pipeline_tiny.npz.
+  reference_experiment/ a ``GenerationExperiment.save`` dump written by the reference (experiment.py:140-167).
+
+    python -m oracle.make_golden reference_trace     # regenerate only the named fixtures
 """
 from __future__ import annotations
 
@@ -162,18 +169,115 @@ def make_perkey_fixture(daam):
     print('perkey', plain.shape)
 
 
-def main():
+def make_reference_trace_fixture(daam):
+    """The scenarios of tests/test_oracle_vs_reference.py under the reference's own trace."""
+    import json
+    import tempfile
+    from pathlib import Path
+    from tests.util import fingerprint
+    fp = lambda t: np.array(fingerprint(t), dtype=np.int64)
+    out = {}
+    # a 2-step generation of the TINY pipeline
+    torch.manual_seed(0)
+    pipe = make_pipeline(TINY_SPEC, dtype=torch.float32, seed=3)
+    with daam.trace(pipe) as tc:
+        pipe(PROMPT, num_inference_steps=2, generator=torch.Generator().manual_seed(11))
+        keys = [k for k, _ in tc.all_heat_maps]
+        out['keys'] = np.array(keys)
+        out['key_shapes'] = np.array([tuple(v.shape) for _, v in tc.all_heat_maps])
+        out['key_fp'] = np.stack([fp(v) for _, v in tc.all_heat_maps])
+        maps = {
+            'global': tc.compute_global_heat_map().heat_maps,
+            'norm': tc.compute_global_heat_map(normalize=True).heat_maps,
+            'f2': tc.compute_global_heat_map(factors=[2]).heat_maps,
+            'l9h0': tc.compute_global_heat_map(layer_idx=9, head_idx=0).heat_maps,
+            'word': tc.compute_global_heat_map().compute_word_heat_map('ball').heatmap,
+        }
+        out['names'] = np.array(list(tc.layer_names))
+    for name, m in maps.items():
+        out[f'{name}_shape'], out[f'{name}_fp'] = np.array(m.shape), fp(m)
+    # the --all-heads sweep over every fifth key, on a second generation under the same trace settings
+    with daam.trace(pipe) as tc:
+        pipe(PROMPT, num_inference_steps=2, generator=torch.Generator().manual_seed(11))
+        sweep = [tc.compute_global_heat_map(layer_idx=l, head_idx=h, normalize=True).heat_maps for f, l, h in keys[::5]]
+    out['sweep_shape'], out['sweep_fp'] = np.array(sweep[0].shape), np.stack([fp(m) for m in sweep])
+    # error messages, token merge indices, _unravel_attn
+    with daam.trace(pipe) as tc:
+        try:
+            tc.compute_global_heat_map()
+        except RuntimeError as e:
+            out['err_no_maps'] = str(e)
+    try:
+        daam.compute_token_merge_indices(pipe.tokenizer, PROMPT, 'zebra')
+    except ValueError as e:
+        out['err_word'] = str(e)
+    merge = {w: daam.compute_token_merge_indices(pipe.tokenizer, PROMPT, w) for w in ['dog', 'red', 'beach']}
+    merge['x@3'] = daam.compute_token_merge_indices(pipe.tokenizer, PROMPT, 'x', word_idx=3)
+    out['merge_indices'] = json.dumps(merge)
+    probs = torch.rand(8, 256, 77, generator=torch.Generator().manual_seed(21))
+    unravelled = daam.trace(pipe).module[0]._unravel_attn(probs)
+    out['unravel_shape'], out['unravel_fp'] = np.array(unravelled.shape), fp(unravelled)
+    # save_heads / load_heads
+    gen = lambda: torch.Generator().manual_seed(2)
+    pipe5, other = make_pipeline(TINY_SPEC, dtype=torch.float32, seed=5), make_pipeline(TINY_SPEC, dtype=torch.float32, seed=6)
+    with tempfile.TemporaryDirectory() as tmp:
+        with daam.trace(pipe5, save_heads=True, data_dir=tmp) as tc:
+            pipe5(PROMPT, num_inference_steps=2, generator=gen())
+            saved = tc.compute_global_heat_map().heat_maps.clone()
+            out['save_layers'] = len(tc.layer_names)
+        names = sorted(p.name for p in Path(tmp).iterdir())
+        out['saved_names'] = np.array(names)
+        out['heads_fp'] = np.stack([fp(torch.load(Path(tmp) / n)) for n in names])
+        with daam.trace(other, load_heads=True, data_dir=tmp) as tc:
+            latents = other(PROMPT, num_inference_steps=2, generator=gen()).latents
+            loaded = tc.compute_global_heat_map().heat_maps.clone()
+    for name, t in [('saved', saved), ('loaded', loaded), ('latents', latents)]:
+        out[f'{name}_shape'], out[f'{name}_fp'] = np.array(t.shape), fp(t)
+    # the 96x96-latent geometry
+    pipe = make_pipeline(TINY96_SPEC, dtype=torch.float32, seed=5)
+    with daam.trace(pipe) as tc:
+        assert tc.latent_hw == 9216
+        pipe(PROMPT, num_inference_steps=2, generator=torch.Generator().manual_seed(13))
+        out['keys96'] = np.array([k for k, _ in tc.all_heat_maps])
+        out['key96_shapes'] = np.array([tuple(v.shape) for _, v in tc.all_heat_maps])
+        out['key96_fp'] = np.stack([fp(v) for _, v in tc.all_heat_maps])
+        g = tc.compute_global_heat_map(normalize=True).heat_maps
+    out['norm96_shape'], out['norm96_fp'] = np.array(g.shape), fp(g)
+    np.savez_compressed(os.path.join(OUT, 'reference_trace.npz'), **out)
+    print('reference_trace', len(keys), 'keys', len(names), 'saved heads')
+
+
+def make_reference_experiment_fixture(daam):
+    """A GenerationExperiment dump written by the reference, with the heat map it holds."""
+    import PIL.Image
+    dst = os.path.join(OUT, 'reference_experiment')
+    os.makedirs(dst, exist_ok=True)
+    maps = torch.rand(6, 16, 16, generator=torch.Generator().manual_seed(4))
+    img = PIL.Image.new('RGB', (16, 16), (10, 20, 30))
+    cwd = os.getcwd()
+    os.chdir(dst)     # the dump pickles its path: keep it relative
+    try:
+        daam.GenerationExperiment(img, maps, 'a red ball', seed=3, id='q1', path='.').save(heat_maps=False)
+    finally:
+        os.chdir(cwd)
+    np.save(os.path.join(dst, 'global_heat_map.npy'), maps.numpy())
+    print('reference_experiment', sorted(os.listdir(os.path.join(dst, 'q1'))))
+
+
+FIXTURES = {'layers': make_layers, 'finalize': make_finalize, 'pipeline_tiny': make_pipeline_fixture,
+            'pipeline_tiny96': make_pipeline96_fixture, 'perkey': make_perkey_fixture,
+            'reference_trace': make_reference_trace_fixture, 'reference_experiment': make_reference_experiment_fixture}
+
+
+def main(names=None):
     warnings.filterwarnings('ignore', category=FutureWarning)
     os.makedirs(OUT, exist_ok=True)
     os.environ.setdefault('XDG_CACHE_HOME', '/tmp/daam_cache')
     torch.set_num_threads(1)   # fixtures must not depend on the thread count
     daam = load_reference()
-    make_layers(daam)
-    make_finalize(daam)
-    make_pipeline_fixture(daam)
-    make_pipeline96_fixture(daam)
-    make_perkey_fixture(daam)
+    for name in names or FIXTURES:
+        FIXTURES[name](daam)
 
 
 if __name__ == '__main__':
-    main()
+    main(sys.argv[1:])

@@ -1,7 +1,7 @@
 """Pins the oracle against the committed golden vectors (outputs of the verbatim reference, oracle/make_golden.py).
 
-Runs everywhere (the GPU box has no /root/reference). Same-machine bit-equality with the live reference is
-tests/test_oracle_vs_reference.py; here the tolerance only absorbs CPU-ISA-dependent summation order."""
+Bit-equality with the reference, on one CPU thread, is tests/test_oracle_vs_reference.py; here the tolerance only
+absorbs summation order that depends on the CPU's instruction set and thread count."""
 import numpy as np
 import pytest
 import torch

@@ -12,6 +12,18 @@ def golden(name):
     return np.load(os.path.join(GOLDEN, name + '.npz'), allow_pickle=False)
 
 
+def fingerprint(t):
+    """Exact, order-independent digest of a float32 tensor's bits: [sum of the bit patterns, position-weighted sum].
+
+    Integer sums are exact in any order, so bit-equal tensors have equal fingerprints on every machine, and a change to
+    any one element changes both sums. It lets a fixture pin tensors too large to store."""
+    t = torch.as_tensor(t).detach().cpu().contiguous()
+    assert t.dtype == torch.float32, t.dtype
+    bits = t.view(torch.int32).to(torch.int64).flatten()
+    weight = torch.arange(bits.numel(), dtype=torch.int64) % 251 + 1
+    return [int(bits.sum()), int((bits * weight).sum())]
+
+
 def oracle_layer_maps(q, k, heads, scale, steps=1):
     """Oracle rows a3+a4 (+a6 summed over `steps` identical calls) for q [B, hw, C], k [B, 77, C]: [N*H, 77, hw] fp32.
 
