@@ -14,7 +14,8 @@
 //                           loads the accumulator;
 //                ldst mode: coalesced 128-byte load / add / store per warp and token, straight from registers.
 // Warp roles: 0-3 epilogue, 4 TMA producer (one elected thread), 5 TMEM allocator + MMA issuer (one thread).
-// Persistent: every CTA walks a contiguous chunk of the launch's tiles; up to 2 CTAs per SM (256 TMEM columns each).
+// Persistent: CTA b of a grid of G takes the launch's tiles b, b + G, b + 2G, ... (K-chunked launches: a contiguous range
+// of equal weight); up to 2 CTAs per SM (256 TMEM columns each).
 //
 // fp32 projections (the reference's default dtype for SD-1.x/2.x, daam/run/generate.py:205) take the same kernel in
 // "split" form. Tensor cores have no fp32 operand type and a plain kind::tf32 product would drop 13 mantissa bits, so
@@ -264,14 +265,22 @@ accumulate_mma_kernel(const __grid_constant__ MmaParams MP) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gen + kOperandBytes + kPBytes + 128);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  int first, count;
-  if constexpr (!kChunked) {                           // equal tiles: contiguous ranges of per / per + 1 tiles
-    const int per = P.total_tiles / gridDim.x, rem = P.total_tiles % gridDim.x;
-    first = blockIdx.x * per + min((int)blockIdx.x, rem);
-    count = per + ((int)blockIdx.x < rem ? 1 : 0);
-  } else {                                             // tiles of several K-chunk counts: contiguous ranges of equal WEIGHT
+  // The i-th tile of this CTA is first + i * stride.
+  int first, count, stride;
+  if constexpr (!kChunked) {
+    // Equal tiles, interleaved: CTA b takes b, b + G, b + 2G, ... The CTAs of a wave then work on adjacent tiles, i.e.
+    // on adjacent 512-byte pieces of the same accumulator token rows (a tile's reduce-add writes 77 of them, 4 * hw
+    // bytes apart), so the L2 read-modify-writes of a wave sweep contiguous DRAM ranges instead of landing ~4.7 tiles
+    // apart as with contiguous per-CTA ranges (SD-2.1 step 23.1 -> 22.4 us, profiles/r03_ab.json).
+    first = blockIdx.x;
+    stride = gridDim.x;
+    count = (P.total_tiles - first + stride - 1) / stride;
+  } else {
+    // Tiles of several K-chunk counts: contiguous ranges of equal WEIGHT. (Interleaving measured 5 % slower on SD-1.5's
+    // fp32 split form and no faster in fp16, profiles/r03_ab.json.)
     first = tile_at_weight(P, (long long)P.total_weight * blockIdx.x / gridDim.x);
     count = tile_at_weight(P, (long long)P.total_weight * (blockIdx.x + 1) / gridDim.x) - first;
+    stride = 1;
   }
 
   if (threadIdx.x == 0) {
@@ -324,7 +333,7 @@ accumulate_mma_kernel(const __grid_constant__ MmaParams MP) {
     uint8_t* lo = gen + kStages * kStageBytesT;
     int li = 0, j = 0;
     for (int i = 0; i < count; ++i) {
-      const Tile t = decode_tile(P, first + i, li);
+      const Tile t = decode_tile(P, first + i * stride, li);
       const LayerParams& L = P.layer[t.li];
       const int n_chunks = kChunked ? (L.head_dim + 63) >> 6 : 1;
       for (int c = 0; c < n_chunks; ++c, ++j) {
@@ -345,7 +354,7 @@ accumulate_mma_kernel(const __grid_constant__ MmaParams MP) {
     if (lane == 0) {
       int li = 0, j = 0;
       for (int i = 0; i < count; ++i) {
-        const Tile t = decode_tile(P, first + i, li);
+        const Tile t = decode_tile(P, first + i * stride, li);
         const int n_chunks = kChunked ? (P.layer[t.li].head_dim + 63) >> 6 : 1;
         for (int c = 0; c < n_chunks; ++c, ++j) {      // one load iteration = one 64-wide K chunk of one tile
           const int s = j % kStages;
@@ -376,7 +385,7 @@ accumulate_mma_kernel(const __grid_constant__ MmaParams MP) {
     if (lane == 0) {
       int li = 0, j = 0;
       for (int i = 0; i < count; ++i) {
-        const Tile t = decode_tile(P, first + i, li);
+        const Tile t = decode_tile(P, first + i * stride, li);
         const LayerParams& L = P.layer[t.li];
         const int a = i & 1;
         const uint32_t aph = (uint32_t)(i >> 1) & 1u;
@@ -426,7 +435,7 @@ accumulate_mma_kernel(const __grid_constant__ MmaParams MP) {
     const int tid = threadIdx.x;                       // 0..127 == pixel within the tile == TMEM lane
     bool issued = false;
     for (int i = 0; i < count; ++i) {
-      const Tile t = decode_tile(P, first + i, li);
+      const Tile t = decode_tile(P, first + i * stride, li);
       const LayerParams& L = P.layer[t.li];
       const int a = i & 1;
       const uint32_t aph = (uint32_t)(i >> 1) & 1u;
@@ -541,10 +550,11 @@ std::unordered_map<MapKey, CUtensorMap, MapKeyHash>& map_cache() {
 std::mutex g_map_mu;
 
 // {head_dim, heads, rows, prompts} view of a projection; box = [box_rows x one 128-byte swizzle span] of one head (64
-// 16-bit or 32 fp32 dims), 128B-swizzled; columns beyond head_dim are zero-filled.
+// 16-bit or 32 fp32 dims), 128B-swizzled; columns beyond head_dim are zero-filled. `promo`: L2 fill granularity.
 int make_qk_map(const void* ptr, int dtype, int head_dim, int heads, int rows, int prompts, long long s_head,
-                long long s_row, long long s_prompt, int box_rows, CUtensorMap* out) {
-  MapKey key{ptr, s_head, s_row, s_prompt, heads, rows, prompts * 1024 + box_rows, (dtype << 4) | (head_dim << 8)};
+                long long s_row, long long s_prompt, int box_rows, CUtensorMapL2promotion promo, CUtensorMap* out) {
+  MapKey key{ptr, s_head, s_row, s_prompt, heads, rows, prompts * 1024 + box_rows,
+             (dtype << 4) | (head_dim << 8) | ((int)promo << 20)};
   {
     std::lock_guard<std::mutex> lock(g_map_mu);
     auto it = map_cache().find(key);
@@ -562,7 +572,7 @@ int make_qk_map(const void* ptr, int dtype, int head_dim, int heads, int rows, i
                                    : dtype == DAAM_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
                                                         : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   CUresult r = enc(out, type, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_SWIZZLE_128B, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(q/k) failed with CUresult %d", (int)r); return DAAM_E_CUDA; }
   std::lock_guard<std::mutex> lock(g_map_mu);
   if (map_cache().size() > 8192) map_cache().clear();
@@ -622,8 +632,11 @@ int prepare_accumulate_mma(const LaunchParams& p, const DeviceInfo& dev, void* o
   for (int i = 0; i < p.n_layers; ++i) {
     const LayerParams& L = p.layer[i];
     if ((L.dtype == DAAM_F32) != split) { set_error("mixed fp32 / 16-bit layers in one tcgen05 pack"); return DAAM_E_INVALID; }
-    if (int rc = make_qk_map(L.q, L.dtype, L.head_dim, L.heads, L.hw, L.n_prompts, L.qs_head, L.qs_pixel, L.qs_prompt, kTilePixels, &mp.qmap[i])) return rc;
-    if (int rc = make_qk_map(L.k, L.dtype, L.head_dim, L.heads, kTokens, L.n_prompts, L.ks_head, L.ks_token, L.ks_prompt, kTokensPad, &mp.kmap[i])) return rc;
+    // A Q tile reads 128 B of each pixel row (one head) at a 640 / 1280 / 2560-byte row stride: 256-byte L2 fills also
+    // bring in the neighbouring head's 128 B, which the CTA owning the same pixels of that head reads in the same wave
+    // of the interleaved schedule (SD-2.1 step 22.4 -> 22.2 us, profiles/r03_ab.json)
+    if (int rc = make_qk_map(L.q, L.dtype, L.head_dim, L.heads, L.hw, L.n_prompts, L.qs_head, L.qs_pixel, L.qs_prompt, kTilePixels, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, &mp.qmap[i])) return rc;
+    if (int rc = make_qk_map(L.k, L.dtype, L.head_dim, L.heads, kTokens, L.n_prompts, L.ks_head, L.ks_token, L.ks_prompt, kTokensPad, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, &mp.kmap[i])) return rc;
     if (int rc = make_acc_map(L.acc, L.hw, L.n_prompts * L.heads * kTokens, &mp.amap[i])) return rc;
     chunked = chunked || L.head_dim > 64;
   }
